@@ -5,7 +5,7 @@ One "step" = one ``ModelInference.infer`` over one synthetic 854x476, T=50 video
 (BASELINE.json configs[1]): trajectories, cos-sims, anchor re-tracking, occlusion.  1 query-point = one
 row of ``infer`` output (T-frame trajectory + T-frame occlusion mask), SURVEY.md 8d.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 * ``value``  : whole-job query-points/s, inputs resident in HBM, device-timed (CUDA events), max over ranks.
 * ``e2e``    : same metric through the public API with HOST buffers: pinned query points H2D, result D2H
@@ -16,6 +16,10 @@ row of ``infer`` output (T-frame trajectory + T-frame occlusion mask), SURVEY.md
 
 N > 1 (torchrun, one rank per GPU): video-parallel -- every rank tracks its own video of the same shape
 (BASELINE configs[2] style), no data-path collective; weak scaling.
+
+``--dump-outputs DIR`` writes what ``infer`` returned in the last timed step (rank 0) as ``DIR/trajectories.npy``
+(N x T x 2 px, float32) and ``DIR/occlusion.npy`` (N x T, float32 0 / 1).  The inputs are seeded, so two builds run with
+the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -31,6 +35,7 @@ import torch
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the source tree as it found it (it may be read-only)
 
 H, W = 476, 854
 GEO_H, GEO_W = 67, 121
@@ -59,7 +64,14 @@ def parse():
     ap.add_argument("--second-head", type=int, default=1, help="0: skip the extra timing with the mixed-sign head")
     ap.add_argument("--multi", type=int, default=1, help="0: skip the config 3 / 4 / 5 blocks (bench_multi.py)")
     ap.add_argument("--config3-vit", type=int, default=1, help="0: config 3 without the ViT stage (tracker + delta-DINO only)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (--impl b200)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return args
 
 
 def synth_video_features(T, C, device, seed, noise):
@@ -322,6 +334,24 @@ def workload_name(args):
 
 
 # ------------------------------------------------------------------------------------------ product arm
+DUMP_BYTES = 60_000_000   # array bytes of one dump: with the .npy headers, under 64 MB
+
+
+def dump_outputs(out_dir, outputs):
+    """``outputs``: {name: tensor with one row per query point} -> out_dir/<name>.npy in float32.  Above DUMP_BYTES in all,
+    a fixed seeded sample of the rows (ascending) is written instead, with its row indices as query_rows.npy."""
+    import numpy as np
+    rows = next(iter(outputs.values())).shape[0]
+    row_bytes = sum(4 * t[0].numel() for t in outputs.values())
+    if rows * row_bytes > DUMP_BYTES:
+        keep = torch.randperm(rows, generator=torch.Generator().manual_seed(0))[:DUMP_BYTES // (row_bytes + 4)].sort().values
+        outputs = {k: t[keep.to(t.device)] for k, t in outputs.items()}
+        outputs["query_rows"] = keep
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def run_b200(args):
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -382,7 +412,7 @@ def run_b200(args):
     t_wall0 = time.perf_counter()
     e0.record()
     for _ in range(args.steps):
-        step_resident()
+        last = step_resident()
     e1.record()
     torch.cuda.synchronize()
     t_wall1 = time.perf_counter()
@@ -393,6 +423,8 @@ def run_b200(args):
     prof = _lib.profile_collect()
     _lib.profile_enable(False)
     clocks = sampler.stop(t_wall0, t_wall1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"trajectories": last[0], "occlusion": last[1]})
 
     # ---- e2e: host buffers, H2D + D2H inside the timed region
     torch.cuda.synchronize()

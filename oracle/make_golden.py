@@ -6,6 +6,8 @@ Test infrastructure (see ``oracle/__init__.py``).  Inputs come from ``oracle/syn
 (seeded, regenerable); outputs are whatever the unmodified reference code under
 ``/root/reference`` returns on CPU behind the three shims of ``oracle/ref_harness.py``.
 """
+import hashlib
+import json
 import os
 import sys
 
@@ -15,7 +17,8 @@ import torch
 from . import ref_harness, synth
 from . import delta_dino as od
 
-GOLDEN_DIR = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
 
 # name: geometry / sizes / seeds of every tracker+inference case
 TRACK_CASES = {
@@ -385,6 +388,53 @@ def gen_vit_case(name, cfg=VIT_CASE):
     print(name, tuple(feats.shape), float(feats.abs().max()))
 
 
+def train_case_arrays(cfg=TRAIN_CASE):
+    """Every input ``gen_train_case`` gives the reference, by name."""
+    geo, feats, video, head, dsd, (pts, src, tgt, fs), labels = train_case_inputs(cfg)
+    out = dict(features=feats, video=video, points=pts, source_frames=src, target_frames=tgt, frames_set=fs, labels=labels)
+    out.update({"head." + k: v for k, v in head.items()})
+    out.update({"delta_dino." + k: v for k, v in dsd.items()})
+    return {k: v.numpy() for k, v in out.items()}
+
+
+def cycle_case_arrays(cfg=CYC_CASE):
+    """Every input ``gen_cycle_case`` gives the reference, by name."""
+    geo, feats, head, fg, (pts, src, tgt, fs) = cyc_case_inputs(cfg)
+    out = dict(features=feats, foreground=fg, points=pts, source_frames=src, target_frames=tgt, frames_set=fs)
+    out.update({"head." + k: v for k, v in head.items()})
+    return {k: v.numpy() for k, v in out.items()}
+
+
+def array_digest(a):
+    """sha256 of an array's dtype, shape and bytes: equal digests = bit-identical arrays."""
+    a = np.ascontiguousarray(a)
+    h = hashlib.sha256(f"{a.dtype.str} {a.shape} ".encode())
+    h.update(a.tobytes())
+    return h.hexdigest()
+
+
+def surface_digest(surface):
+    """sha256 of the drop-in surface (tools/dropin_surface.py) in a canonical JSON form."""
+    return hashlib.sha256(json.dumps(surface, sort_keys=True).encode()).hexdigest()
+
+
+def reference_digests(golden_dir=GOLDEN_DIR):
+    """What the CPU suite checks without the reference (tests/test_golden_regen_cpu.py, tests/test_dropin_surface.py):
+    digests of the inputs the training-step and cycle-consistency cases give the reference and of the fixtures in
+    ``golden_dir`` that it returned for them, and the digest of the drop-in surface extracted from the reference's
+    sources.  Run right after those fixtures were generated."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("dropin_surface", os.path.join(ROOT, "tools", "dropin_surface.py"))
+    tool = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(tool)
+    out = {"dropin_surface": surface_digest(tool.surface(ref_harness.REFERENCE_ROOT))}
+    for name, inputs in (("train_small", train_case_arrays()), ("cycle_small", cycle_case_arrays())):
+        fixture = np.load(os.path.join(golden_dir, name + ".npz"))
+        out[name] = {"inputs": {k: array_digest(v) for k, v in sorted(inputs.items())},
+                     "outputs": {k: array_digest(fixture[k]) for k in sorted(fixture.files)}}
+    return out
+
+
 def main():
     os.makedirs(GOLDEN_DIR, exist_ok=True)
     torch.set_num_threads(8)
@@ -398,6 +448,8 @@ def main():
     gen_vit_case("vit_small")
     gen_train_case("train_small")
     gen_cycle_case("cycle_small")
+    with open(os.path.join(GOLDEN_DIR, "reference_digests.json"), "w") as f:
+        json.dump(reference_digests(), f, indent=1)
 
 
 if __name__ == "__main__":

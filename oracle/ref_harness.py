@@ -2,8 +2,8 @@
 
 Test infrastructure (see ``oracle/__init__.py``).  Usable only where
 ``/root/reference`` exists (the build container); never on the GPU box.  Used by
-``oracle/make_golden.py`` to produce ``tests/golden/*`` and by the CPU tests
-that re-validate the oracle against the reference when it is present.
+``oracle/make_golden.py`` to produce ``tests/golden/*`` (the fixtures and the
+digests that pin them, ``reference_digests.json``).
 
 Shims (SURVEY.md 8c) -- none of them touches the arithmetic of the hot path:
   1. ``antialiased_cnns.BlurPool`` (third-party, adobe/antialiased-cnns, not

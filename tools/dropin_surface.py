@@ -1,6 +1,6 @@
 """Extracts the attribute surface the reference's own entry points touch on ``Tracker`` / ``ModelInference`` objects and
-writes tests/golden/dropin_surface.json (run in the build container; the CPU test re-derives it when the reference tree is
-present and otherwise checks the committed copy).
+writes tests/golden/dropin_surface.json (needs the reference tree; ``python -m oracle.make_golden`` records the digest of the
+extraction, which the CPU test checks the committed copy against).
 
 Walked (AssafSinger94/dino-tracker @ 5b0f2b0): inference_grid.py, inference_benchmark.py (variables ``model``,
 ``model_inference``), dino_tracker.py::get_model / train_setup (``model``), models/model_inference.py (``self.model`` /
