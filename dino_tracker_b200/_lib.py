@@ -193,11 +193,12 @@ def profile_collect():
 
 
 def infer_stats():
-    """{anchor-phase maps, finished by the exact-window path, re-done by the full-map path, pipeline} of the last infer."""
-    a = (ctypes.c_longlong * 5)()
-    check(load().dinotrk_infer_last_stats(a, 5), "infer_last_stats")
+    """{anchor-phase maps, finished by the exact-window path, re-done by the full-map path, pipeline} of the last infer,
+    plus the re-done maps queued by the certificate and the exact-window cells by the part count of their token box."""
+    a = (ctypes.c_longlong * 8)()
+    check(load().dinotrk_infer_last_stats(a, 8), "infer_last_stats")
     return {"anchor_maps": int(a[0]), "exact_window": int(a[1]), "full_map": int(a[2]), "pipeline": "exact-window" if a[3] else "full-map",
-            "full_map_by_certificate": int(a[4])}
+            "full_map_by_certificate": int(a[4]), "exact_window_cells_by_parts": {p: int(a[3 + p]) for p in (2, 3, 4)}}
 
 
 def launch_count():

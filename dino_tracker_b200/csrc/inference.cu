@@ -423,7 +423,8 @@ constexpr int XW_PROBE_MAPS = 4096;   // size of the probe chunk (automatic pipe
 struct XwAsync {
   int state;                                   // 0: not created, 1: ready, -1: failed
   cudaEvent_t sample[XW_RING], done[XW_RING], freed[XW_RING];
-  int* host_cnt;                               // pinned: [XW_RING][2] queue totals / uncertified + [16] phase-A uncertified counts
+  int* host_cnt;                               // pinned: [XW_RING][XW_NCNT] chunk counters (XwChunk::slow_cnt from [n_groups])
+                                               // + [16] phase-A uncertified counts + the smallest token norm
 };
 static XwAsync* xw_async() {
   static PerDev<XwAsync> slots;
@@ -435,13 +436,16 @@ static XwAsync* xw_async() {
       if (cudaEventCreateWithFlags(&xa.done[k], cudaEventDisableTiming) != cudaSuccess) return nullptr;
       if (cudaEventCreateWithFlags(&xa.freed[k], cudaEventDisableTiming) != cudaSuccess) return nullptr;
     }
-    if (cudaHostAlloc(&xa.host_cnt, (2 * XW_RING + 16 + 4) * sizeof(int), cudaHostAllocDefault) != cudaSuccess) return nullptr;
+    if (cudaHostAlloc(&xa.host_cnt, (XW_NCNT * XW_RING + 16 + 4) * sizeof(int), cudaHostAllocDefault) != cudaSuccess) return nullptr;
     xa.state = 1;
   }
   return xa.state == 1 ? &xa : nullptr;
 }
 static int g_xw_path = -1;                     // -1: automatic (DTK_XW or on), 0: full-map path only, 1: exact-window path
-static long long g_infer_stats[5] = {0, 0, 0, 0, 0};   // anchor-phase maps | on the exact-window path | queued | path used | queued by the certificate
+// anchor-phase maps | on the exact-window path | queued | path used | queued by the certificate | exact-window cells whose box
+// has 2, 3, 4 M-parts
+constexpr int INFER_NSTATS = 5 + (XW_PARTS - 1);
+static long long g_infer_stats[INFER_NSTATS] = {};
 
 }  // namespace dtk
 
@@ -457,7 +461,7 @@ int dinotrk_infer_set_path(int path) {
 
 int dinotrk_infer_last_stats(long long* out, int n) {
   DTK_CHECK_ARG(out && n >= 4, "infer_last_stats: need at least 4 slots");
-  for (int i = 0; i < (n < 5 ? n : 5); ++i) out[i] = g_infer_stats[i];
+  for (int i = 0; i < (n < INFER_NSTATS ? n : INFER_NSTATS); ++i) out[i] = g_infer_stats[i];
   return DINOTRK_OK;
 }
 
@@ -679,11 +683,11 @@ int dinotrk_infer(const dinotrk_features* feat, const dinotrk_geom* g,
     x.pinfo = ar.take<int>(ch);
     x.cell_of = ar.take<int>(ch);
     x.slow_list = ar.take<int>(ch);
-    x.box_org = ar.take<int2>((size_t)ch + 2);
+    x.box = ar.take<XwBox>((size_t)ch + 2);
     x.xbox = ar.take<float>((size_t)ch * XW_COLS);
     x.win = ar.take<float>((size_t)ch * 256);
     x.hin = ar.take<int2>(ch);
-    x.slow_cnt = ar.take<int>(gcap + 2);
+    x.slow_cnt = ar.take<int>(gcap + XW_NCNT);
   }
   const int cell_nb = (T + XW_MAX_CELL - 1) / XW_MAX_CELL;
   int* d_cells = ar.take<int>((size_t)N * T * cell_nb * 4 + 16);
@@ -786,27 +790,28 @@ int dinotrk_infer(const dinotrk_features* feat, const dinotrk_geom* g,
     if (xa) {   // reciprocal token norms for the coarse epilogue + the smallest norm of the video (the host reads it below)
       int rcn = launch_xw_rnorms(fv, d_rnorms, d_minnorm, st);
       if (rcn) return rcn;
-      DTK_CUDA(cudaMemcpyAsync(xa->host_cnt + 2 * XW_RING + 16, d_minnorm, sizeof(unsigned), cudaMemcpyDeviceToHost, st));
+      DTK_CUDA(cudaMemcpyAsync(xa->host_cnt + XW_NCNT * XW_RING + 16, d_minnorm, sizeof(unsigned), cudaMemcpyDeviceToHost, st));
     }
     if (xa && n_chunks_A > 0)
-      DTK_CUDA(cudaMemcpyAsync(xa->host_cnt + 2 * XW_RING, d_cntA, (size_t)n_chunks_A * sizeof(int), cudaMemcpyDeviceToHost, st));
+      DTK_CUDA(cudaMemcpyAsync(xa->host_cnt + XW_NCNT * XW_RING, d_cntA, (size_t)n_chunks_A * sizeof(int), cudaMemcpyDeviceToHost, st));
     DTK_CUDA(cudaMemcpyAsync(cnt.data(), d_cnt, (size_t)T * sizeof(int), cudaMemcpyDeviceToHost, st));
     DTK_CUDA(cudaStreamSynchronize(st));  // the one host sync: sizes of the anchor work lists
     if (use_xw) {   // a (near-)zero token anywhere voids the coarse pass's error bound (xwin.cuh: XW_MIN_NORM)
       float mn;
-      memcpy(&mn, xa->host_cnt + 2 * XW_RING + 16, sizeof(float));
+      memcpy(&mn, xa->host_cnt + XW_NCNT * XW_RING + 16, sizeof(float));
       if (!(mn >= XW_MIN_NORM)) use_xw = false;
     }
     if (use_xw && pathsel < 0 && n_chunks_A > 0) {
       // head weights the certificate cannot handle send (almost) every map to the full-map kernels anyway: the trajectory
       // phase just showed it; skip the exact-window attempt then.  (Depends on the weights and the video only.)
       long long unc = 0;
-      for (int k = 0; k < n_chunks_A; ++k) unc += xa->host_cnt[2 * XW_RING + k];
+      for (int k = 0; k < n_chunks_A; ++k) unc += xa->host_cnt[XW_NCNT * XW_RING + k];
       if (unc * 4 > maps_A) use_xw = false;
     }
     long long maps_C = 0;
     for (int a = 0; a < T; ++a) maps_C += (long long)cnt[a] * T;
-    g_infer_stats[0] = maps_C; g_infer_stats[1] = 0; g_infer_stats[2] = 0; g_infer_stats[3] = use_xw ? 1 : 0; g_infer_stats[4] = 0;
+    for (long long& v : g_infer_stats) v = 0;
+    g_infer_stats[0] = maps_C; g_infer_stats[3] = use_xw ? 1 : 0;
     size_t k0 = 0;            // first chunk of the full-map pipeline (> 0 after an exact-window probe)
     bool planned = false;
     if (use_xw) {
@@ -874,8 +879,9 @@ int dinotrk_infer(const dinotrk_features* feat, const dinotrk_geom* g,
       };
       auto finish = [&](size_t j) -> int {
         DTK_CUDA(cudaEventSynchronize(xa->done[j % XW_RING]));
-        const int n_slow = xa->host_cnt[2 * (j % XW_RING)];
-        g_infer_stats[4] += xa->host_cnt[2 * (j % XW_RING) + 1];
+        const int* hc = xa->host_cnt + XW_NCNT * (j % XW_RING);
+        const int n_slow = hc[0];
+        for (int i = 1; i < XW_NCNT; ++i) g_infer_stats[3 + i] += hc[i];   // queued by the certificate, cells by part count
         const ChunkMeta& cm = metas[j];
         const XwSet& x = xr[j % XW_RING];
         const Grp gp = grp_of(j);
@@ -920,7 +926,8 @@ int dinotrk_infer(const dinotrk_features* feat, const dinotrk_geom* g,
         if ((rc = launch_xw_gemm(fv, *g, hi_of(x, cm.used), lo_of(x, cm.used), cm.used, cells, x.xc, st))) return rc;
         if ((rc = launch_xw_head(fv, *g, *hw, cells, x.norm, gp.map0, cm.used, x.out_index, anchors, 2, 0, x.xc, st, cm.n_groups)))
           return rc;
-        DTK_CUDA(cudaMemcpyAsync(xa->host_cnt + 2 * (k % XW_RING), x.xc.slow_cnt + cm.n_groups, 2 * sizeof(int), cudaMemcpyDeviceToHost, st));
+        DTK_CUDA(cudaMemcpyAsync(xa->host_cnt + XW_NCNT * (k % XW_RING), x.xc.slow_cnt + cm.n_groups, XW_NCNT * sizeof(int),
+                                 cudaMemcpyDeviceToHost, st));
         DTK_CUDA(cudaEventRecord(xa->done[k % XW_RING], st));
         if (k == 0 && probing && metas.size() > 1) {   // the probe: wait for it, look at the certificate's verdicts
           if ((rc = finish(0))) return rc;

@@ -126,16 +126,17 @@ int launch_xw_coarse(const FeatView& fv, const void* desc_hi, int desc_rows, con
 // (a) one warp per MAP (lane = tile): global coarse maximum, candidate tiles (max1 >= gmax - 2 eps), ambiguity (some tile's
 //     SECOND value is also within 2 eps: an arg-max candidate whose token is unknown).  Writes the candidate tokens and
 //     pinfo[map] = coarse arg-max token, or -1 - token if the map is ambiguous.
-// (b) one warp per CELL: the lower medians of the unambiguous maps' coarse arg-max row / column give the box centre; a map
-//     fits if every candidate lies within +-XW_SLACK of it.
+// (b) one warp per CELL: a map fits if every candidate lies within +-XW_SLACK of the lower medians of the unambiguous maps'
+//     coarse arg-max row / column.  The cell's box covers the 15 x 15 windows around every fitting candidate: 16 columns
+//     (8 box rows per M-part) when those candidates span <= 2 columns, else 21 (6 rows per part); 2..4 parts.
 constexpr int PLAN_WARPS = 8;
 __global__ void __launch_bounds__(PLAN_WARPS * 32)
 xw_cand_kernel(int n_maps, const float* __restrict__ desc_norm, int n_groups, int n_tiles, const unsigned long long* __restrict__ key1,
                const float* __restrict__ max2, int* __restrict__ cand, int* __restrict__ pinfo, int* __restrict__ slow_cnt) {
   const int lane = threadIdx.x & 31;
   const int gw = blockIdx.x * PLAN_WARPS + (threadIdx.x >> 5), nw = gridDim.x * PLAN_WARPS;
-  if (gw == 0)   // zero the queue counters of this chunk (n_groups per-group counts + the total + the uncertified count)
-    for (int i = lane; i <= n_groups + 1; i += 32) slow_cnt[i] = 0;
+  if (gw == 0)   // zero the counters of this chunk (n_groups per-group queue lengths + XW_NCNT chunk totals)
+    for (int i = lane; i < n_groups + XW_NCNT; i += 32) slow_cnt[i] = 0;
   for (int map = gw; map < n_maps; map += nw) {
     const unsigned long long* k1 = key1 + (size_t)map * n_tiles;
     const float* k2 = max2 + (size_t)map * n_tiles;
@@ -174,7 +175,7 @@ xw_cand_kernel(int n_maps, const float* __restrict__ desc_norm, int n_groups, in
 
 __global__ void __launch_bounds__(PLAN_WARPS * 32)
 xw_cell_kernel(XwCells cells, int w, const int* __restrict__ cand, const int* __restrict__ pinfo, int* __restrict__ stat,
-               int* __restrict__ cell_of, int2* __restrict__ box_org) {
+               int* __restrict__ cell_of, XwBox* __restrict__ box, int* __restrict__ part_cnt) {
   __shared__ short s_r[PLAN_WARPS][XW_MAX_CELL], s_c[PLAN_WARPS][XW_MAX_CELL];
   __shared__ unsigned char s_ok[PLAN_WARPS][XW_MAX_CELL];
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -215,10 +216,12 @@ xw_cell_kernel(XwCells cells, int w, const int* __restrict__ cand, const int* __
         med_c = max(med_c, __shfl_xor_sync(0xffffffffu, med_c, o));
       }
     }
-    int n_fit = 0;
+    // bounding rectangle of the fitting maps' candidates (within +-XW_SLACK of the medians: at most 7 x 7 tokens)
+    int n_fit = 0, r_lo = INT_MAX, r_hi = INT_MIN, c_lo = INT_MAX, c_hi = INT_MIN;
     for (int r = lane; r < m; r += 32) {
       const int map = row0 + r;
       bool fit = s_ok[wid][r] != 0;
+      int mr_lo = INT_MAX, mr_hi = INT_MIN, mc_lo = INT_MAX, mc_hi = INT_MIN;
       if (fit) {
         const int4 cd = __ldg(reinterpret_cast<const int4*>(cand) + map);
         const int ct[4] = {cd.x, cd.y, cd.z, cd.w};
@@ -227,15 +230,30 @@ xw_cell_kernel(XwCells cells, int w, const int* __restrict__ cand, const int* __
           if (ct[q] >= 0) {
             const int tr = ct[q] / w, tc_ = ct[q] - tr * w;
             fit = fit && abs(tr - med_r) <= XW_SLACK && abs(tc_ - med_c) <= XW_SLACK;
+            mr_lo = min(mr_lo, tr); mr_hi = max(mr_hi, tr); mc_lo = min(mc_lo, tc_); mc_hi = max(mc_hi, tc_);
           }
       }
       stat[map] = fit ? 0 : 1;
       n_fit += fit ? 1 : 0;
+      if (fit) { r_lo = min(r_lo, mr_lo); r_hi = max(r_hi, mr_hi); c_lo = min(c_lo, mc_lo); c_hi = max(c_hi, mc_hi); }
     }
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1) n_fit += __shfl_xor_sync(0xffffffffu, n_fit, o);
-    if (lane == 0)
-      box_org[cell] = n_fit > 0 ? make_int2(med_r - XW_BOX / 2, med_c - XW_BOX / 2) : make_int2(0, INT_MIN);
+    for (int o = 16; o > 0; o >>= 1) {
+      n_fit += __shfl_xor_sync(0xffffffffu, n_fit, o);
+      r_lo = min(r_lo, __shfl_xor_sync(0xffffffffu, r_lo, o)); r_hi = max(r_hi, __shfl_xor_sync(0xffffffffu, r_hi, o));
+      c_lo = min(c_lo, __shfl_xor_sync(0xffffffffu, c_lo, o)); c_hi = max(c_hi, __shfl_xor_sync(0xffffffffu, c_hi, o));
+    }
+    if (lane == 0) {
+      XwBox b{0, 0, 0, 0, 0};
+      if (n_fit > 0) {   // the rectangle widened by the window's half side (7) on every side: 15..21 rows and columns
+        const int height = r_hi - r_lo + 15;
+        const bool wide = c_hi - c_lo + 15 > XW_NARROW;
+        const int rows = wide ? XW_ROWS_WIDE : XW_ROWS_NARROW;
+        b = XwBox{r_lo - 7, c_lo - 7, (short)(wide ? XW_BOX : XW_NARROW), (short)height, (short)((height + rows - 1) / rows)};
+        atomicAdd(part_cnt + b.parts - 2, 1);
+      }
+      box[cell] = b;
+    }
     __syncwarp();
   }
 }
@@ -254,28 +272,30 @@ int launch_xw_plan(const XwCells& cells, const float* desc_norm, int n_groups, c
   DTK_LAUNCHED();
   grid = cdiv(cells.n_cells, PLAN_WARPS);
   if (grid > 148 * 8) grid = 148 * 8;
-  xw_cell_kernel<<<grid, PLAN_WARPS * 32, 0, st>>>(cells, g.w, xc.cand, xc.pinfo, xc.stat, xc.cell_of, xc.box_org);
+  xw_cell_kernel<<<grid, PLAN_WARPS * 32, 0, st>>>(cells, g.w, xc.cand, xc.pinfo, xc.stat, xc.cell_of, xc.box,
+                                                   xc.slow_cnt + n_groups + 2);
   DTK_LAUNCHED();
   return DINOTRK_OK;
 }
 
 // ====================================================================================================== 3. exact box GEMM
 // Persistent, warp-specialised (same roles as tc_gemm_kernel).  One "tile" = one cell.  The BOX TOKENS are the UMMA M
-// operand (4 parts of 6 box rows = 126 of 128 rows) and the cell's descriptors the N operand (64 or 128 columns): a cell
-// of T = 50 maps fills 50 of 64 columns, where descriptors-as-rows filled 50 of 128 rows.  D[part][token][map] in TMEM
-// (4 x NB columns; two cells in flight for NB = 64), split precision (lo*hi + hi*lo + hi*hi per K step, in the full-map
-// GEMM's order).  A K-block of the descriptors (hi, lo) is loaded once and used by the four parts; the box rows arrive as
-// 4-D TMA boxes {64 channels, 21 columns, 6 rows, 1 frame} of the [T][h][w][C] feature video, zero-filled outside the
-// token grid.  Epilogue: TMEM lane = box token, so for every map the 32 lanes of a warp write 32 consecutive floats of
-// its accumulator row -- coalesced without a transpose.
+// operand and the cell's descriptors the N operand (64 or 128 columns): a cell of T = 50 maps fills 50 of 64 columns, where
+// descriptors-as-rows filled 50 of 128 rows.  The cell's box (XwBox) comes in M-parts of 128 rows: 8 box rows of a 16-wide
+// box (2 or 3 parts) or 6 rows of a 21-wide one (126 of 128 rows, 3 or 4 parts).  D[part][token][map] in TMEM (a slot of
+// 4 x NB columns whatever the cell's part count; two cells in flight for NB = 64), split precision (lo*hi + hi*lo + hi*hi
+// per K step, in the full-map GEMM's order).  A K-block of the descriptors (hi, lo) is loaded once and used by the cell's
+// parts; the box rows arrive as 4-D TMA boxes {64 channels, 16 columns, 8 rows, 1 frame} or {64, 21, 6, 1} of the
+// [T][h][w][C] feature video, zero-filled outside the token grid (rows of the last part past the box are computed and
+// dropped).  Epilogue: TMEM lane = box token, so for every map the 32 lanes of a warp write consecutive floats of its
+// accumulator row -- coalesced without a transpose.
 template <int NB>
 struct XwCfg {
   static constexpr int kBK = 64;                            // fp16 elements per 128-byte swizzle row
-  static constexpr int kTokBytes = 128 * 128;               // one operand half (hi or lo) of a token tile: 128 rows, 126 written
+  static constexpr int kTokBytes = 128 * 128;               // hi or lo half of a token tile: 128 rows (126 used by a 21-wide box)
   static constexpr int kTokStage = 2 * kTokBytes, kTokStages = NB == 64 ? 5 : 4;
-  static constexpr int kTokTx = 2 * XW_PART_TOK * 128;
-  static constexpr int kLastRows = XW_BOX - (XW_PARTS - 1) * XW_PART_ROWS;     // the last part holds 3 box rows, not 6
-  static constexpr int kTokTxLast = 2 * kLastRows * XW_BOX * 128;
+  static constexpr int kTokTxNarrow = 2 * XW_ROWS_NARROW * XW_NARROW * 128, kTokTxWide = 2 * XW_ROWS_WIDE * XW_BOX * 128;
+  static_assert(XW_ROWS_NARROW * XW_NARROW <= 128 && XW_ROWS_WIDE * XW_BOX <= 128, "an M-part is at most 128 tokens");
   static constexpr int kDescBytes = NB * 128;               // one operand half of the descriptor K-block
   static constexpr int kDescStage = 2 * kDescBytes, kDescStages = 2;
   static constexpr int kSmem = kDescStages * kDescStage + kTokStages * kTokStage + 256;
@@ -296,9 +316,9 @@ __device__ __forceinline__ void tma_load_4d(const CUtensorMap* m, uint64_t* bar,
 template <int NB>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 xw_gemm_kernel(const __grid_constant__ CUtensorMap tmD_hi, const __grid_constant__ CUtensorMap tmD_lo,
-               const __grid_constant__ CUtensorMap tmT_hi, const __grid_constant__ CUtensorMap tmT_lo,
-               const __grid_constant__ CUtensorMap tmL_hi, const __grid_constant__ CUtensorMap tmL_lo, XwCells cells,
-               const int2* __restrict__ box_org, float* __restrict__ xbox, int K) {
+               const __grid_constant__ CUtensorMap tmN_hi, const __grid_constant__ CUtensorMap tmN_lo,
+               const __grid_constant__ CUtensorMap tmW_hi, const __grid_constant__ CUtensorMap tmW_lo, XwCells cells,
+               const XwBox* __restrict__ box, float* __restrict__ xbox, int K) {
   using Cfg = XwCfg<NB>;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw;
@@ -319,8 +339,8 @@ xw_gemm_kernel(const __grid_constant__ CUtensorMap tmD_hi, const __grid_constant
   const int KB = (K + Cfg::kBK - 1) / Cfg::kBK;
 
   if (warp == 0 && lane == 0) {
-    tc::prefetch_tmap(&tmD_hi); tc::prefetch_tmap(&tmD_lo); tc::prefetch_tmap(&tmT_hi); tc::prefetch_tmap(&tmT_lo);
-    tc::prefetch_tmap(&tmL_hi); tc::prefetch_tmap(&tmL_lo);
+    tc::prefetch_tmap(&tmD_hi); tc::prefetch_tmap(&tmD_lo); tc::prefetch_tmap(&tmN_hi); tc::prefetch_tmap(&tmN_lo);
+    tc::prefetch_tmap(&tmW_hi); tc::prefetch_tmap(&tmW_lo);
     for (int s = 0; s < Cfg::kDescStages; ++s) { tc::mbar_init(&d_full[s], 1); tc::mbar_init(&d_empty[s], 1); }
     for (int s = 0; s < Cfg::kTokStages; ++s) { tc::mbar_init(&t_full[s], 1); tc::mbar_init(&t_empty[s], 1); }
     for (int s = 0; s < 2; ++s) { tc::mbar_init(&tfull[s], 1); tc::mbar_init(&tempty[s], 4); }
@@ -337,8 +357,12 @@ xw_gemm_kernel(const __grid_constant__ CUtensorMap tmD_hi, const __grid_constant
     if (tc::elect_one()) {
       int ds = 0, dph = 0, ts = 0, tph = 0;
       for (int cell = blockIdx.x; cell < cells.n_cells; cell += gridDim.x) {
-        const int2 org = box_org[cell];
-        if (org.y == INT_MIN) continue;            // every map of the cell takes the full-map path
+        const XwBox bx = box[cell];
+        if (bx.parts == 0) continue;               // every map of the cell takes the full-map path
+        const bool wide = bx.width == XW_BOX;
+        const CUtensorMap* tm_hi = wide ? &tmW_hi : &tmN_hi;
+        const CUtensorMap* tm_lo = wide ? &tmW_lo : &tmN_lo;
+        const int rows = wide ? XW_ROWS_WIDE : XW_ROWS_NARROW, tx = wide ? Cfg::kTokTxWide : Cfg::kTokTxNarrow;
         const int drow = cells.row0[cell], frame = cells.frame[cell];
         for (int kb = 0; kb < KB; ++kb) {
           const int k0 = kb * Cfg::kBK;
@@ -348,18 +372,12 @@ xw_gemm_kernel(const __grid_constant__ CUtensorMap tmD_hi, const __grid_constant
           tc::tma_load_2d(&tmD_hi, &d_full[ds], sd, k0, drow);
           tc::tma_load_2d(&tmD_lo, &d_full[ds], sd + Cfg::kDescBytes, k0, drow);
           if (++ds == Cfg::kDescStages) { ds = 0; dph ^= 1; }
-          for (int part = 0; part < XW_PARTS; ++part) {
+          for (int part = 0; part < bx.parts; ++part) {
             tc::mbar_wait(&t_empty[ts], tph ^ 1);
             uint8_t* st = t_ring + ts * Cfg::kTokStage;
-            if (part < XW_PARTS - 1) {
-              tc::mbar_expect_tx(&t_full[ts], Cfg::kTokTx);
-              tc::tma_load_4d(&tmT_hi, &t_full[ts], st, k0, org.y, org.x + part * XW_PART_ROWS, frame);
-              tc::tma_load_4d(&tmT_lo, &t_full[ts], st + Cfg::kTokBytes, k0, org.y, org.x + part * XW_PART_ROWS, frame);
-            } else {   // only the box rows that exist (this kernel runs at the L2 -> shared-memory bandwidth)
-              tc::mbar_expect_tx(&t_full[ts], Cfg::kTokTxLast);
-              tc::tma_load_4d(&tmL_hi, &t_full[ts], st, k0, org.y, org.x + part * XW_PART_ROWS, frame);
-              tc::tma_load_4d(&tmL_lo, &t_full[ts], st + Cfg::kTokBytes, k0, org.y, org.x + part * XW_PART_ROWS, frame);
-            }
+            tc::mbar_expect_tx(&t_full[ts], tx);
+            tc::tma_load_4d(tm_hi, &t_full[ts], st, k0, bx.col, bx.row + part * rows, frame);
+            tc::tma_load_4d(tm_lo, &t_full[ts], st + Cfg::kTokBytes, k0, bx.col, bx.row + part * rows, frame);
             if (++ts == Cfg::kTokStages) { ts = 0; tph ^= 1; }
           }
         }
@@ -369,14 +387,15 @@ xw_gemm_kernel(const __grid_constant__ CUtensorMap tmD_hi, const __grid_constant
     // ===================== MMA issuer =====================
     int ds = 0, dph = 0, ts = 0, tph = 0, it = 0;
     for (int cell = blockIdx.x; cell < cells.n_cells; cell += gridDim.x) {
-      if (box_org[cell].y == INT_MIN) continue;
+      const int parts = box[cell].parts;
+      if (parts == 0) continue;
       const int buf = it % Cfg::kAccBufs, use = it / Cfg::kAccBufs;
       tc::mbar_wait(&tempty[buf], (use & 1) ^ 1);
       tc::fence_after_sync();
       for (int kb = 0; kb < KB; ++kb) {
         tc::mbar_wait(&d_full[ds], dph);
         const uint32_t sd = tc::smem_u32(d_ring + ds * Cfg::kDescStage);
-        for (int part = 0; part < XW_PARTS; ++part) {
+        for (int part = 0; part < parts; ++part) {
           tc::mbar_wait(&t_full[ts], tph);
           tc::fence_after_sync();
           if (tc::elect_one()) {
@@ -393,7 +412,7 @@ xw_gemm_kernel(const __grid_constant__ CUtensorMap tmD_hi, const __grid_constant
               tc::mma_ss<false>(tmem_d, t_hi, d_hi, Cfg::kIdesc, 1u);
             }
             tc::mma_commit(&t_empty[ts]);
-            if (part == XW_PARTS - 1) {
+            if (part == parts - 1) {
               tc::mma_commit(&d_empty[ds]);
               if (kb == KB - 1) tc::mma_commit(&tfull[buf]);
             }
@@ -410,16 +429,18 @@ xw_gemm_kernel(const __grid_constant__ CUtensorMap tmD_hi, const __grid_constant
     const int quad = warp & 3;
     int it = 0;
     for (int cell = blockIdx.x; cell < cells.n_cells; cell += gridDim.x) {
-      if (box_org[cell].y == INT_MIN) continue;
+      const XwBox bx = box[cell];
+      if (bx.parts == 0) continue;
       const int m = cells.m[cell], map0 = cells.row0[cell];
+      const int part_tok = (bx.width == XW_BOX ? XW_ROWS_WIDE : XW_ROWS_NARROW) * bx.width;
       const int buf = it % Cfg::kAccBufs, use = it / Cfg::kAccBufs;
       tc::mbar_wait(&tfull[buf], use & 1);
       tc::fence_after_sync();
       const int tok = quad * 32 + lane;
 #pragma unroll 1
-      for (int part = 0; part < XW_PARTS; ++part) {
-        const int col = part * XW_PART_TOK + tok;
-        const bool ok = tok < XW_PART_TOK && col < XW_BOX * XW_BOX;
+      for (int part = 0; part < bx.parts; ++part) {
+        const int col = part * part_tok + tok;
+        const bool ok = tok < part_tok && col < bx.height * bx.width;
         const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + buf * Cfg::kAccCols + part * NB;
         float* dst = xbox + (size_t)map0 * XW_COLS + col;
 #pragma unroll 1
@@ -455,18 +476,17 @@ int launch_xw_gemm(const FeatView& fv, const dinotrk_geom& g, const void* desc_h
   DTK_CHECK_ARG(fv.C % 8 == 0 && cells.max_m <= XW_MAX_CELL, "exact-window GEMM: bad sizes");
   const bool small = cells.max_m <= 64;
   const int nb = small ? 64 : 128;
-  CUtensorMap tD_hi, tD_lo, tT_hi, tT_lo, tL_hi, tL_lo;
+  CUtensorMap tD_hi, tD_lo, tN_hi, tN_lo, tW_hi, tW_lo;
   int rc;
   if ((rc = make_tmap_2d(&tD_hi, desc_hi, desc_rows, fv.C, nb, 64, TMAP_F16))) return rc;
   if ((rc = make_tmap_2d(&tD_lo, desc_lo, desc_rows, fv.C, nb, 64, TMAP_F16))) return rc;
   const uint64_t dims[4] = {(uint64_t)fv.C, (uint64_t)g.w, (uint64_t)g.h, (uint64_t)fv.T};
   const uint64_t strides[3] = {(uint64_t)fv.C * 2, (uint64_t)g.w * fv.C * 2, (uint64_t)fv.P * fv.C * 2};
-  const uint32_t box[4] = {64, XW_BOX, XW_PART_ROWS, 1};
-  if ((rc = make_tmap_4d(&tT_hi, fv.hi, dims, strides, box, TMAP_F16))) return rc;
-  if ((rc = make_tmap_4d(&tT_lo, fv.lo, dims, strides, box, TMAP_F16))) return rc;
-  const uint32_t box_last[4] = {64, XW_BOX, (uint32_t)XwCfg<64>::kLastRows, 1};
-  if ((rc = make_tmap_4d(&tL_hi, fv.hi, dims, strides, box_last, TMAP_F16))) return rc;
-  if ((rc = make_tmap_4d(&tL_lo, fv.lo, dims, strides, box_last, TMAP_F16))) return rc;
+  const uint32_t box_n[4] = {64, XW_NARROW, XW_ROWS_NARROW, 1}, box_w[4] = {64, XW_BOX, XW_ROWS_WIDE, 1};
+  if ((rc = make_tmap_4d(&tN_hi, fv.hi, dims, strides, box_n, TMAP_F16))) return rc;
+  if ((rc = make_tmap_4d(&tN_lo, fv.lo, dims, strides, box_n, TMAP_F16))) return rc;
+  if ((rc = make_tmap_4d(&tW_hi, fv.hi, dims, strides, box_w, TMAP_F16))) return rc;
+  if ((rc = make_tmap_4d(&tW_lo, fv.lo, dims, strides, box_w, TMAP_F16))) return rc;
   static PerDev<bool> attr_dev;
   bool& attr = attr_dev.get();
   if (!attr) {
@@ -480,9 +500,9 @@ int launch_xw_gemm(const FeatView& fv, const dinotrk_geom& g, const void* desc_h
   const int grid = cells.n_cells < sms ? cells.n_cells : sms;
   ProfRange pr(PROF_XW_GEMM, st);
   if (small)
-    xw_gemm_kernel<64><<<grid, TC_THREADS, XwCfg<64>::kSmem, st>>>(tD_hi, tD_lo, tT_hi, tT_lo, tL_hi, tL_lo, cells, xc.box_org, xc.xbox, fv.C);
+    xw_gemm_kernel<64><<<grid, TC_THREADS, XwCfg<64>::kSmem, st>>>(tD_hi, tD_lo, tN_hi, tN_lo, tW_hi, tW_lo, cells, xc.box, xc.xbox, fv.C);
   else
-    xw_gemm_kernel<128><<<grid, TC_THREADS, XwCfg<128>::kSmem, st>>>(tD_hi, tD_lo, tT_hi, tT_lo, tL_hi, tL_lo, cells, xc.box_org, xc.xbox, fv.C);
+    xw_gemm_kernel<128><<<grid, TC_THREADS, XwCfg<128>::kSmem, st>>>(tD_hi, tD_lo, tN_hi, tN_lo, tW_hi, tW_lo, cells, xc.box, xc.xbox, fv.C);
   DTK_LAUNCHED();
   return DINOTRK_OK;
 }
@@ -652,7 +672,7 @@ __device__ __forceinline__ void xw_refine(const XhParams& hp, const float2* __re
 constexpr int XWIN_PITCH = 256;
 __global__ void __launch_bounds__(256)
 xw_window_kernel(int n_maps, int h, int w, int P, int n_tiles, const float* __restrict__ norms, const float* __restrict__ desc_norm,
-                 const int* __restrict__ cell_frame, const int* __restrict__ cell_of, const int2* __restrict__ box_org,
+                 const int* __restrict__ cell_frame, const int* __restrict__ cell_of, const XwBox* __restrict__ box,
                  const int* __restrict__ stat, const int* __restrict__ cand, const unsigned long long* __restrict__ key1,
                  const float* __restrict__ max2, const float* __restrict__ xbox, float* __restrict__ win, int2* __restrict__ hin) {
   const int lane = threadIdx.x & 31;
@@ -663,7 +683,7 @@ xw_window_kernel(int n_maps, int h, int w, int P, int n_tiles, const float* __re
       continue;
     }
     const int cell = cell_of[map];
-    const int2 org = box_org[cell];
+    const XwBox bx = box[cell];
     const float* fn = norms + (size_t)cell_frame[cell] * P;
     const float* xr = xbox + (size_t)map * XW_COLS;
     const float dn = desc_norm[map];
@@ -676,7 +696,7 @@ xw_window_kernel(int n_maps, int h, int w, int P, int n_tiles, const float* __re
     for (int q = 0; q < XW_MAX_CAND; ++q)
       if (ct[q] >= 0) {
         const int tr = ct[q] / w, tcn = ct[q] - tr * w;
-        const float v = fmaxf(__fdiv_rn(__ldg(xr + xw_col(tr - org.x, tcn - org.y)), fmaxf(__fmul_rn(dn, __ldg(fn + ct[q])), 1e-8f)), 0.f);
+        const float v = fmaxf(__fdiv_rn(__ldg(xr + xw_col(tr - bx.row, tcn - bx.col, bx.width)), fmaxf(__fmul_rn(dn, __ldg(fn + ct[q])), 1e-8f)), 0.f);
         if (v > best || (v == best && ct[q] < amax)) { best = v; amax = ct[q]; }
       }
     const int arow = amax / w, acol = amax - arow * w;
@@ -698,7 +718,7 @@ xw_window_kernel(int n_maps, int h, int w, int P, int n_tiles, const float* __re
       const int r = arow - 7 + y, c = acol - 7 + x;
       float v = 0.f;
       if (y < XWM && x < XWM && r >= 0 && r < h && c >= 0 && c < w) {
-        v = fmaxf(__fdiv_rn(__ldg(xr + xw_col(r - org.x, c - org.y)), fmaxf(__fmul_rn(dn, __ldg(fn + r * w + c)), 1e-8f)), 0.f);
+        v = fmaxf(__fdiv_rn(__ldg(xr + xw_col(r - bx.row, c - bx.col, bx.width)), fmaxf(__fmul_rn(dn, __ldg(fn + r * w + c)), 1e-8f)), 0.f);
         if (!(abs(r - arow) <= 3 && abs(c - acol) <= 3)) mout = fmaxf(mout, v);
       }
       win[(size_t)map * XWIN_PITCH + i] = v;
@@ -829,7 +849,7 @@ int launch_xw_head(const FeatView& fv, const dinotrk_geom& g, const dinotrk_head
   {
     int wgrid = cdiv(n_maps, 8);
     if (wgrid > sms * 8) wgrid = sms * 8;
-    xw_window_kernel<<<wgrid, 256, 0, st>>>(n_maps, g.h, g.w, hp.P, hp.n_tiles, fv.norms, desc_norm, cells.frame, xc.cell_of, xc.box_org,
+    xw_window_kernel<<<wgrid, 256, 0, st>>>(n_maps, g.h, g.w, hp.P, hp.n_tiles, fv.norms, desc_norm, cells.frame, xc.cell_of, xc.box,
                                             xc.stat, xc.cand, xc.key1, xc.max2, xc.xbox, xc.win, xc.hin);
     DTK_LAUNCHED();
   }
@@ -898,10 +918,10 @@ size_t xw_chunk_bytes(int chunk_maps, int max_cells, int n_tiles, int gcap) {
   size_t b = 0;
   b += align_up(ch * n_tiles * 8, 256) + align_up(ch * n_tiles * 4, 256);              // key1, max2
   b += align_up(ch * XW_MAX_CAND * 4, 256) + 4 * align_up(ch * 4, 256);                // cand, stat, pinfo, cell_of, slow_list
-  b += align_up((size_t)max_cells * 8, 256);                                           // box_org
+  b += align_up((size_t)max_cells * sizeof(XwBox), 256);                               // box
   b += align_up(ch * XW_COLS * 4, 256);                                                // xbox
   b += align_up(ch * 256 * 4, 256) + align_up(ch * 8, 256);                            // win, hin
-  b += align_up((size_t)(gcap + 2) * 4, 256);                                          // slow_cnt
+  b += align_up((size_t)(gcap + XW_NCNT) * 4, 256);                                    // slow_cnt
   return b + 2048;
 }
 

@@ -11,11 +11,14 @@
 //                    <= XW_EPS for every token (fp16 rounding of both operands + TMEM accumulation, see DESIGN.md).
 //   2. plan          per map: the tokens that can be the exact arg-max (coarse >= max - 2 XW_EPS); a map whose candidates
 //                    are not all tile maxima is "ambiguous".  Maps come in CELLS = the <= 128 source frames of one (query,
-//                    anchor frame) pair: their arg-maxes cluster around the query's position in the anchor frame, so one
-//                    21 x 21 token box around the cell's median arg-max holds every map's window.
+//                    anchor frame) pair: their arg-maxes cluster around the query's position in the anchor frame.  A map
+//                    fits if its candidates lie within +-XW_SLACK of the cell's median arg-max; the cell's box is the
+//                    bounding rectangle of the fitting maps' candidates widened by 7 tokens on every side (so it holds every
+//                    fitting map's 15 x 15 window): 15..21 rows by 16 columns (column extent <= 1) or 21 columns.
 //   3. exact GEMM    per cell, the fp32-faithful split-precision contraction (lo*hi + hi*lo + hi*hi, same operation
-//                    sequence as the full-map GEMM) of the cell's descriptors against the box's 441 tokens only:
-//                    5.4 % of the map.  Raw accumulators go to a [map][448] buffer (1.8 KB per map instead of 32 KB).
+//                    sequence as the full-map GEMM) of the cell's descriptors against the box's tokens only (at most 441,
+//                    5.4 % of the map; 240..256 for a cell whose members agree to one token).  Raw accumulators go to a
+//                    [map][448] buffer, row-major with the cell's box width as pitch (1.8 KB per map instead of 32 KB).
 //   4. head          two kernels, one warp per map each: (a) exact arg-max among the candidates + the exact 15 x 15 window
 //                    + m_out (dependent gathers: many warps per SM), (b) refiner, softmax sums on the 11 x 11 box, certificate
 //                    with the bound from (1); writes the track point.
@@ -28,20 +31,28 @@
 namespace dtk {
 
 constexpr float XW_EPS = 1.1e-3f;     // bound on |coarse - exact| in cosine units (2^-10 + accumulation, rounded up)
-constexpr int XW_BOX = 21;            // box side (tokens); windows of maps whose arg-max lies within +-3 of the centre fit
+constexpr int XW_BOX = 21;            // largest box side (tokens): windows of maps whose candidates lie within +-3 of the centre
 constexpr int XW_SLACK = 3;
-constexpr int XW_PARTS = 4, XW_PART_ROWS = 6;                    // 4 M-parts of 6 box rows (126 tokens = 126 UMMA rows of 128)
-constexpr int XW_PART_TOK = XW_PART_ROWS * XW_BOX;
-constexpr int XW_COLS = 448;                                     // accumulator row pitch per map (441 box tokens, row-major)
+constexpr int XW_NARROW = 16;         // box width when the fitting candidates span <= 2 columns
+// One UMMA M-part = 128 rows: 8 box rows of a 16-wide box (128 tokens) or 6 rows of a 21-wide one (126 tokens)
+constexpr int XW_ROWS_NARROW = 8, XW_ROWS_WIDE = 6;
+constexpr int XW_PARTS = 4;           // most parts of a box (21 x 21: ceil(21 / 6)); a cell's TMEM slot holds XW_PARTS x NB columns
+constexpr int XW_COLS = 448;                                     // accumulator row pitch per map (<= 441 box tokens, row-major)
 constexpr int XW_MAX_CELL = 128;      // maps (source frames) per cell = UMMA N (64 or 128)
 constexpr int XW_MAX_CAND = 4;
 constexpr float XW_MIN_NORM = 1e-4f;  // the coarse pass forms acc / (|d| |F|) without the reference's max(|d| |F|, 1e-8) clamp: both
                                       // norms must be >= 1e-4 (smaller descriptor norms -> ambiguous map, smaller token norms
                                       // anywhere in the video -> the whole call takes the full-map pipeline)
 constexpr int XW_TILE = 128;          // tokens per coarse key (the coarse GEMM's 8 epilogue warps cover 128 columns each)
+constexpr int XW_NCNT = 2 + (XW_PARTS - 1);   // chunk counters after the per-group queue lengths (see XwChunk::slow_cnt)
 
-// column of box token (by, bx) in a map's accumulator row
-__host__ __device__ inline int xw_col(int by, int bx) { return by * XW_BOX + bx; }
+// column of box token (by, bx) in a map's accumulator row (box of `width` columns)
+__host__ __device__ inline int xw_col(int by, int bx, int width) { return by * width + bx; }
+
+struct __align__(16) XwBox {   // a cell's token box: first row and column, width (16 or 21), height (15..21), M-parts
+  int row, col;                 // (2..4; 0: no map of the cell fits, the cell is skipped)
+  short width, height, parts;
+};
 
 struct XwChunk {          // device buffers of one chunk in flight (all sized for chunk_maps maps)
   unsigned long long* key1;   // [maps][n_tiles]  coarse maximum of a XW_TILE-token tile << 32 | (0x7fffffff - first token)
@@ -50,11 +61,12 @@ struct XwChunk {          // device buffers of one chunk in flight (all sized fo
   int* pinfo;                 // [maps] coarse arg-max token, or -1 - token for an ambiguous map (plan scratch)
   int* stat;                  // [maps] 0: exact-window path, 1: full-map path
   int* cell_of;               // [maps] cell index
-  int2* box_org;              // [cells] (first box row, first box column); x = INT_MIN: skip the cell
+  XwBox* box;                 // [cells] token box; parts = 0: no map of the cell fits, every map takes the full-map path
   float* xbox;                // [maps][XW_COLS] raw split-precision accumulators of the box tokens
   float* win;                 // [maps][256] exact 15 x 15 windows ([15][16] floats, zero outside the map)
   int2* hin;                  // [maps] (exact first arg-max token or -1, bits of m_out)
-  int* slow_cnt;              // [n_groups + 1] per group count of queued maps; [n_groups] = total
+  int* slow_cnt;              // [n_groups + XW_NCNT] per group count of queued maps; [n_groups] = total, [n_groups + 1] =
+                              // queued by the certificate, [n_groups + 2 + i] = cells whose box has 2 + i parts
   int* slow_list;             // [maps] group g's queue lives at [grp_map0[g], grp_map0[g] + slow_cnt[g])
 };
 

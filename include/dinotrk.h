@@ -179,8 +179,9 @@ int dinotrk_infer_set_overlap(int mode);
  *      showed that the head's certificate fails for more than a quarter of the maps (ill-conditioned refiner weights);
  *      the DTK_XW environment variable (0 / 1) overrides.
  * dinotrk_infer_last_stats (n >= 4 slots): {anchor-phase maps, maps finished by the exact-window path, maps re-done by the
- * full-map path, pipeline used[, of the re-done maps: those queued by the head's certificate rather than by the plan]} of
- * the last dinotrk_infer call that ran the anchor phase. */
+ * full-map path, pipeline used[, of the re-done maps: those queued by the head's certificate rather than by the plan[,
+ * exact-window cells whose token box took 2, 3, 4 GEMM parts]]} of the last dinotrk_infer call that ran the anchor phase
+ * (n >= 5 returns the certificate count, n >= 8 also the part counts). */
 int dinotrk_infer_set_path(int path);
 int dinotrk_infer_last_stats(long long* out, int n);
 int dinotrk_infer(const dinotrk_features* feat, const dinotrk_geom* g,
